@@ -4,6 +4,7 @@
 
     python bench.py --gpus N --steps K --warmup W            (N>1: launched under torch.distributed.run)
     python bench.py --impl reference ...                     (CPU arm: the oracle port of the reference path)
+    python bench.py ... --dump-outputs DIR                   (also write the last timed step's outputs as DIR/*.npy)
 
 A "step" is ONE denoising step of the batch: one UNet evaluation at batch 16 (8 images x [uncond, cond])
 through the CUDA engine + the fused sampler update.  50 PLMS steps cost 51 UNet evaluations
@@ -257,6 +258,17 @@ def gemm_roofline(prog, pk):
                 note="events bracket each launch individually (serialised, includes launch gaps)")
 
 
+def write_dumps(out_dir, arrays, limit=64 << 20):
+    """DIR/<name>.npy per array; the workloads' outputs are a few MB, far below `limit` (64 MB in all)."""
+    import numpy as np
+    total = sum(a.nbytes for a in arrays.values())
+    if total > limit:
+        raise SystemExit(f"--dump-outputs: {total} bytes of outputs exceed the {limit}-byte limit")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -269,7 +281,15 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-roofline", action="store_true")
     ap.add_argument("--no-graph", action="store_true", help="launch kernels individually (for ncu launch lists)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned (rank 0's shard) as DIR/<name>.npy, float32: x_prev "
+                         "(the sampler's x_{t-1}), eps (the UNet output; [uncond; cond] when guided) and, for PLMS, e_t "
+                         "(the guided eps the sampler keeps); every input is seeded, so equal arguments give equal inputs")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the CUDA path's outputs (--impl b200)")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     if args.impl == "reference":
         return run_reference_arm(args)
@@ -343,7 +363,8 @@ def main():
     ctx = c_host.to(dev) if c_host is not None else None
     nxt = torch.empty_like(x)
     e_t = torch.empty_like(x)
-    old = [torch.randn_like(x) for _ in range(3)]
+    gen = torch.Generator(device=dev).manual_seed(44)     # PLMS history and the eta > 0 noise: same draws on every run
+    old = [torch.randn(x.shape, device=dev, generator=gen) for _ in range(3)]
 
     def step(i, x_in, nxt, ctx_dev):
         """One denoising step in the loop's steady state (PLMS: multistep order 4, 47 of the 50 steps): one UNet evaluation
@@ -355,9 +376,10 @@ def main():
             t = torch.full((UB,), int(ts[k]), device=dev, dtype=torch.long)
             eps = qnn(torch.cat([x_in, x_in]) if guided else x_in, t, ctx_dev)
         a_t, a_prev = alpha[k]
-        noise = torch.randn_like(x_in) if sigma[k] != 0.0 else None
+        noise = torch.randn(x_in.shape, device=dev, generator=gen) if sigma[k] != 0.0 else None
         samplers._step(x_in, eps, nxt, a_t=a_t, a_prev=a_prev, sigma=sigma[k], cfg_scale=CFG_SCALE, coef=coef,
                        olds=tuple(old[:olds_n]) + (None,) * (3 - olds_n), eps_out=e_t if olds_n else None, noise=noise)
+        return eps
 
     def barrier():
         if dist is not None:
@@ -373,11 +395,16 @@ def main():
         torch.cuda.profiler.start()    # no-op unless run under `ncu --profile-from-start off` (profiles/: launch list)
         e0.record()
         for i in range(args.steps):
-            step(args.warmup + i, x, nxt, ctx)
+            eps = step(args.warmup + i, x, nxt, ctx)
         e1.record()
         barrier()
         torch.cuda.profiler.stop()
     ms = e0.elapsed_time(e1)
+    # the e2e pass below reuses these buffers: copy the last timed step's outputs now
+    dumps = None
+    if args.dump_outputs:
+        dumps = dict(x_prev=nxt, eps=eps, **(dict(e_t=e_t) if olds_n else {}))
+        dumps = {k: v.float().cpu().numpy() for k, v in dumps.items()}
     launches = L.qd_launch_count() - launches0
     prog = qnn.program(x, ctx, cfg_dedup=True) if cfg_dedup else qnn.program(torch.cat([x, x]) if guided else x, ctx)
     # with a CUDA graph the kernels replay without passing through the C ABI: count them from the program
@@ -458,6 +485,8 @@ def main():
         torch.set_num_threads(host_threads())
         cb = cpu_baseline(ckpt)
         line["cpu_baseline"] = cb
+    if dumps is not None:
+        write_dumps(args.dump_outputs, dumps)
     print(json.dumps(line))
     if dist is not None:
         dist.destroy_process_group()

@@ -81,53 +81,6 @@ def test_forward_without_cuda_fails_loudly():
         qnn.model.conv_in(g["x"])
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/qdiff"), reason="reference checkout not present (GPU box)")
-@pytest.mark.parametrize("name", ["sd_tiny_w4a8_sm16", "ddim_w4a8_split"])
-def test_wraps_the_references_own_module_objects(name):
-    """Drop-in claim: qdiff_b200.QuantModel wraps the REFERENCE's UNetModel / Model instances (dispatch by class
-    name), and resume_cali_model consumes the checkpoint written by the reference for that very model."""
-    import sys
-    import tempfile
-    import types
-    stub = tempfile.mkdtemp()
-    os.makedirs(os.path.join(stub, "omegaconf"))
-    open(os.path.join(stub, "omegaconf", "__init__.py"), "w").write("")
-    open(os.path.join(stub, "omegaconf", "listconfig.py"), "w").write("class ListConfig(list):\n    pass\n")
-    sys.path[:0] = [stub, "/root/reference"]
-    try:
-        import qdiff_b200 as qd
-        g = load_case(name)
-        p, q = g["params"], g["qcfg"]
-        if g["family"] == "ddim":
-            from ddim.models.diffusion import Model
-            ns = types.SimpleNamespace
-            cfg = ns(model=ns(type="simple", in_channels=p["in_channels"], out_ch=p["out_ch"], ch=p["ch"], ch_mult=p["ch_mult"],
-                              num_res_blocks=p["num_res_blocks"], attn_resolutions=p["attn_resolutions"], dropout=0.0,
-                              resamp_with_conv=True),
-                     data=ns(image_size=p["resolution"]), diffusion=ns(num_diffusion_timesteps=1000),
-                     split_shortcut=p["split_shortcut"])
-            model = Model(cfg)
-        else:
-            from ldm.modules.diffusionmodules.openaimodel import UNetModel
-            model = UNetModel(**p["unet"])
-            model.split = p.get("split", False)
-        wq = {'n_bits': q["weight_bit"], 'channel_wise': True, 'scale_method': 'max'}
-        aq = {'n_bits': q["act_bit"], 'symmetric': q["a_sym"], 'channel_wise': False, 'scale_method': 'max',
-              'leaf_param': True}
-        qnn = qd.QuantModel(model=model, weight_quant_params=wq, act_quant_params=aq, sm_abit=q["sm_abit"])
-        qd.resume_cali_model(qnn, g["ckpt"], None, quant_act=True)
-        kinds = {type(m).__name__ for m in qnn.modules()}
-        assert "QuantModule" in kinds and ("QuantResBlock" in kinds or "QuantResnetBlock" in kinds)
-        w = dict(qnn.named_parameters())
-        k0 = next(k for k in g["ckpt"] if k.endswith("conv_in.weight") or k.endswith("input_blocks.0.0.weight"))
-        assert torch.equal(w[k0].detach(), g["ckpt"][k0])
-    finally:
-        sys.path.remove(stub)
-        sys.path.remove("/root/reference")
-        for mod in [m for m in sys.modules if m.split(".")[0] in ("ldm", "ddim", "qdiff", "omegaconf")]:
-            del sys.modules[mod]
-
-
 def test_pack_int4_roundtrip_and_limits():
     """ops.pack_int4: unsigned nibbles + per-row zero point reproduce the zero-point-free codes; rows that do not fit
     4 bits (W8 layers) are refused so the builder falls back to the s8 layout."""
